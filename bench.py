@@ -2,6 +2,7 @@
 """bench.py -- denoising steps/sec on 256x256 tiles of the 30m decoder U-Net (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|reference-gpu] [--tiles B] [--size S]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -45,6 +46,25 @@ def igemm_gflop(size: int) -> float:
     """FLOPs executed by the tcgen05 implicit-GEMM launches in one forward (everything except first/last conv, linears)."""
     # BASELINE.md Appendix F: 6->64 first conv 0.453, 64->1 last conv 0.075, linears 0.003 at 256^2
     return (GFLOP_PER_STEP_256 - 0.453 - 0.075 - 0.003) * (size / 256.0) ** 2
+
+
+DUMP_LIMIT_BYTES = 60 << 20     # all arrays of one dump, so the files (with their .npy headers) stay under 64 MB
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Write each tensor as <out_dir>/<name>.npy in float32, so two builds run with the same arguments (hence the same
+    seeded inputs) can be compared output for output.  A tensor larger than its share of DUMP_LIMIT_BYTES is stored as
+    every k-th element of its flattened form, the smallest k that fits: the same elements on every run."""
+    import numpy as np
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    limit = DUMP_LIMIT_BYTES // len(arrays)
+    for name, t in arrays.items():
+        t = t.detach().float()
+        stride = -(-t.numel() * 4 // limit)
+        if stride > 1:
+            t = t.reshape(-1)[::stride]
+        np.save(d / f"{name}.npy", t.cpu().numpy())
 
 
 # ----------------------------------------------------------------------------------------------------- clocks
@@ -640,7 +660,14 @@ def main():
                          "(configs[2]: one 1664^2 canvas, strong scaling) | export (configs[3]-shaped 9344^2 canvas)")
     ap.add_argument("--solve-steps", type=int, default=SOLVE_STEPS, help="denoising steps per tile (canvas workloads)")
     ap.add_argument("--tile-batch", type=int, default=4, help="tiles solved together per launch (canvas workloads)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the denoised tiles of the last timed step (rank 0) as "
+                         "DIR/sample.npy, float32 [tiles, 1, size, size]; a strided sample if above 60 MiB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "tiles"):
+        ap.error("--dump-outputs is implemented for the default arm (--impl ours --workload tiles)")
     if args.warmup < 3:
         args.warmup = 3
 
@@ -701,8 +728,10 @@ def main():
         return plan, solves
 
     def run_plan(plan, solves):
+        out = None
         for n in plan:
-            solves[n].run(noise_d, cond_d)
+            out = solves[n].run(noise_d, cond_d)
+        return out
 
     wplan, wsolves = make_solves(args.warmup)
     plan, solves = make_solves(args.steps)
@@ -717,9 +746,12 @@ def main():
     torch.cuda.synchronize()
     with ClockSampler(local_rank) as clk:
         e0.record()
-        run_plan(plan, solves)         # exactly K timed steps
+        last = run_plan(plan, solves)  # exactly K timed steps
         e1.record()
         torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0:
+        # `last` is the solver's state buffer: the e2e and roofline passes below overwrite it
+        dump_outputs(args.dump_outputs, {"sample": last})
     if world > 1:
         dist.barrier()
     ms = e0.elapsed_time(e1)
