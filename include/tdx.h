@@ -37,7 +37,7 @@ extern "C" {
 const char* tdx_last_error(void);
 /* Library + device probe: fills sm count, compute capability; fails if the device is not sm_100. */
 int tdx_device_info(int* sm_count, int* cc_major, int* cc_minor);
-/* sizeof() of the public structs (0: TdxOutSpec, 1: TdxIgemmDesc, 2: TdxConvInDesc, 3: TdxConvOutDesc, 4: TdxEmbedBlock, 5: TdxEmbedDesc, 6: TdxAttnDesc) so bindings can verify their layout. */
+/* sizeof() of the public structs (0: TdxOutSpec, 1: TdxIgemmDesc, 2: TdxConvInDesc, 3: TdxConvOutDesc, 4: TdxEmbedBlock, 5: TdxEmbedDesc, 6: TdxAttnDesc, 7: TdxIm2colDesc, 8: TdxConvOutGuidedDesc) so bindings can verify their layout. */
 int tdx_abi_sizeof(int which);
 
 /* ------------------------------------------------------------------------------------------------------------------
@@ -158,6 +158,19 @@ typedef struct TdxConvOutDesc {
   float* x0_prev;          /* fp32 NCHW solver history, read+written (requires sched_coef) */
 } TdxConvOutDesc;
 int tdx_conv_out_run(const TdxConvOutDesc* desc, void* stream);
+/* The same launch with two-model autoguidance (EDM2 autoguidance; sample_diffusion_base.py:105-110,
+ * sample_diffusion_decoder.py:112-117) applied to the convolution's result before the update:
+ *     F_m = conv3x3(x_raw) ;  F = F_g + s*(F_m - F_g)   (separately rounded sub, mul, add)
+ *     x0  = c_skip*sample + c_out*F ; sample' = r*sample + (1-r)*x0 + k*(x0 - x0_prev) ; x0_prev = x0
+ * F_g (guide_out) is the guide model's output, fp32 NCHW [n_img][c_out][H][W], e.g. written earlier in the same program
+ * by the guide's own last convolution in plain model_out mode.  base.sched_coef is required and points at FIVE device
+ * floats {c_skip, c_out, r, k, s}: the guidance scale lives in the table, so a recorded program can change it without
+ * being rebuilt.  base.model_out (optional) receives the combined F. */
+typedef struct TdxConvOutGuidedDesc {
+  TdxConvOutDesc base;
+  const float* guide_out;
+} TdxConvOutGuidedDesc;
+int tdx_conv_out_guided_run(const TdxConvOutGuidedDesc* desc, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------------
  * Embedding path (EDMUnet2D.compute_embeddings, models/edm_unet.py:145-159, + the per-block modulation vector of
@@ -304,6 +317,7 @@ int tdx_program_add_conv_in(TdxProgram* p, const TdxConvInDesc* d);
 int tdx_program_add_im2col(TdxProgram* p, const TdxIm2colDesc* d);
 int tdx_program_add_igemm(TdxProgram* p, const TdxIgemmDesc* d);
 int tdx_program_add_conv_out(TdxProgram* p, const TdxConvOutDesc* d);
+int tdx_program_add_conv_out_guided(TdxProgram* p, const TdxConvOutGuidedDesc* d);
 int tdx_program_add_embed(TdxProgram* p, const TdxEmbedDesc* d);
 int tdx_program_add_attn(TdxProgram* p, const TdxAttnDesc* d);
 int tdx_program_num_launches(const TdxProgram* p);
@@ -312,7 +326,7 @@ int tdx_program_run(TdxProgram* p, int use_graph, void* stream);
 /* Capture + instantiate + upload the graph without running it (keeps one-time costs out of timed regions). */
 int tdx_program_instantiate(TdxProgram* p, void* stream);
 /* Eager run with a CUDA event pair around every launch: ms_per_launch[i] = device time of launch i (in program
- * order, tdx_program_num_launches entries); kinds[i] = 0 conv_in, 1 igemm, 2 conv_out, 3 embed, 4 attn, 5 im2col.  Synchronises. */
+ * order, tdx_program_num_launches entries); kinds[i] = 0 conv_in, 1 igemm, 2 conv_out (guided or not), 3 embed, 4 attn, 5 im2col.  Synchronises. */
 int tdx_program_profile(TdxProgram* p, float* ms_per_launch, int32_t* kinds, void* stream);
 int tdx_program_destroy(TdxProgram* p);
 

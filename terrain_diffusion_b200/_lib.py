@@ -52,6 +52,10 @@ class TdxConvOutDesc(C.Structure):
     ]
 
 
+class TdxConvOutGuidedDesc(C.Structure):
+    _fields_ = [("base", TdxConvOutDesc), ("guide_out", C.c_void_p)]
+
+
 class TdxEmbedBlock(C.Structure):
     _fields_ = [("weight", C.c_void_p), ("cvec", C.c_void_p), ("c_out", C.c_int32), ("_pad", C.c_int32)]
 
@@ -70,7 +74,7 @@ class TdxAttnDesc(C.Structure):
 
 
 ABI_STRUCTS = [TdxOutSpec, TdxIgemmDesc, TdxConvInDesc, TdxConvOutDesc, TdxEmbedBlock, TdxEmbedDesc, TdxAttnDesc,
-               TdxIm2colDesc]
+               TdxIm2colDesc, TdxConvOutGuidedDesc]
 
 OUT_NONE, OUT_RAW, OUT_SILU, OUT_PNORM_SILU = 0, 1, 2, 3
 SP_SAME, SP_DOWN2, SP_UP2 = 0, 1, 2
@@ -109,8 +113,8 @@ def _declare(l: C.CDLL) -> None:
         if l.tdx_abi_sizeof(i) != C.sizeof(st):
             raise TdxError(f"ABI mismatch for {st.__name__}: C {l.tdx_abi_sizeof(i)} vs ctypes {C.sizeof(st)}")
     for name, desc in (("tdx_conv_in_run", TdxConvInDesc), ("tdx_conv_out_run", TdxConvOutDesc),
-                       ("tdx_embed_run", TdxEmbedDesc), ("tdx_attn_run", TdxAttnDesc),
-                       ("tdx_im2col_run", TdxIm2colDesc)):
+                       ("tdx_conv_out_guided_run", TdxConvOutGuidedDesc), ("tdx_embed_run", TdxEmbedDesc),
+                       ("tdx_attn_run", TdxAttnDesc), ("tdx_im2col_run", TdxIm2colDesc)):
         fn = getattr(l, name)
         fn.restype = C.c_int
         fn.argtypes = [C.POINTER(desc), C.c_void_p]
@@ -173,7 +177,8 @@ def _declare(l: C.CDLL) -> None:
     l.tdx_program_create.restype = C.c_int
     l.tdx_program_create.argtypes = [C.POINTER(C.c_void_p)]
     for name, desc in (("tdx_program_add_conv_in", TdxConvInDesc), ("tdx_program_add_igemm", TdxIgemmDesc),
-                       ("tdx_program_add_conv_out", TdxConvOutDesc), ("tdx_program_add_embed", TdxEmbedDesc),
+                       ("tdx_program_add_conv_out", TdxConvOutDesc),
+                       ("tdx_program_add_conv_out_guided", TdxConvOutGuidedDesc), ("tdx_program_add_embed", TdxEmbedDesc),
                        ("tdx_program_add_attn", TdxAttnDesc), ("tdx_program_add_im2col", TdxIm2colDesc)):
         fn = getattr(l, name)
         fn.restype = C.c_int

@@ -134,6 +134,7 @@ extern "C" int tdx_abi_sizeof(int which) {
     case 5: return (int)sizeof(TdxEmbedDesc);
     case 6: return (int)sizeof(TdxAttnDesc);
     case 7: return (int)sizeof(TdxIm2colDesc);
+    case 8: return (int)sizeof(TdxConvOutGuidedDesc);
     default: return -1;
   }
 }

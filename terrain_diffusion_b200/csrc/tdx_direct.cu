@@ -332,6 +332,7 @@ struct ConvOutParams {
   const float* coef;
   float* sample;
   float* x0_prev;
+  const float* guide_out;   // GUIDED: the guide model's F_g (fp32 NCHW); the guidance scale is coef[4]
 };
 
 // One DPM-Solver++(2M) update in the EDM closed form (scheduler/dpmsolver.py:419-561; SURVEY.md Appendix B).
@@ -344,7 +345,9 @@ __device__ __forceinline__ void sched_update(float x, float f, float x0p, float 
 
 // Block = 128 threads = 32 pixels x 4 sub-threads; sub-thread s accumulates channel groups s, s+4, ... so four times as
 // many 16-byte loads are in flight; the partial sums are combined with two warp shuffles.  COUT = 1 (decoder) or 8.
-template <int COUT>
+// GUIDED: two-model autoguidance before the update, F = F_g + s*(F_m - F_g) with F_m = conv3x3(x), separately rounded
+// in the reference's order (sample_diffusion_base.py:110, sample_diffusion_decoder.py:117); model_out receives F.
+template <int COUT, bool GUIDED>
 __global__ void __launch_bounds__(128) conv_out_kernel(const ConvOutParams p) {
   extern __shared__ float ws[];  // [tap][c][COUT]
   const int C = p.C8 * 8;
@@ -364,6 +367,13 @@ __global__ void __launch_bounds__(128) conv_out_kernel(const ConvOutParams p) {
     float acc[COUT];
 #pragma unroll
     for (int j = 0; j < COUT; ++j) acc[j] = 0.f;
+    // the guide's output is issued with the activation loads, not after the reduction
+    float fg[GUIDED ? COUT : 1];
+    if (GUIDED) {
+#pragma unroll
+      for (int oc = 0; oc < COUT; ++oc)
+        fg[oc] = (inb && sub == 0 && oc < p.cout) ? __ldg(p.guide_out + ((size_t)img * p.cout + oc) * plane + pix) : 0.f;
+    }
     if (COUT == 1 && p.C8 == 8) {
       // the decoder's 64 -> 1 case: all 18 loads of a thread are issued before the first is used (the generic loop
       // below walks taps and groups with data-dependent control flow: one L2 latency after the other).  Out-of-image
@@ -425,12 +435,14 @@ __global__ void __launch_bounds__(128) conv_out_kernel(const ConvOutParams p) {
       acc[j] += __shfl_xor_sync(0xffffffff, acc[j], 16);
     }
     if (!inb || sub != 0) continue;
-    float cs = 0.f, co = 0.f, r = 0.f, k = 0.f;
+    float cs = 0.f, co = 0.f, r = 0.f, k = 0.f, gs = 1.f;
     if (p.coef) { cs = __ldg(p.coef); co = __ldg(p.coef + 1); r = __ldg(p.coef + 2); k = __ldg(p.coef + 3); }
+    if (GUIDED) gs = __ldg(p.coef + 4);
 #pragma unroll
     for (int oc = 0; oc < COUT; ++oc) {
       if (oc >= p.cout) break;
       const size_t idx = ((size_t)img * p.cout + oc) * plane + pix;
+      if (GUIDED) acc[oc] = __fadd_rn(fg[oc], __fmul_rn(gs, __fsub_rn(acc[oc], fg[oc])));
       if (p.model_out) p.model_out[idx] = acc[oc];
       if (p.coef) {
         float xn, x0;
@@ -448,8 +460,10 @@ int direct_prepare() {
   if (first_use_on_device(seen)) {
     TDX_CHECK_CUDA(cudaFuncSetAttribute(conv_in_kernel<6>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
     TDX_CHECK_CUDA(cudaFuncSetAttribute(conv_in_kernel<12>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    TDX_CHECK_CUDA(cudaFuncSetAttribute(conv_out_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    TDX_CHECK_CUDA(cudaFuncSetAttribute(conv_out_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    TDX_CHECK_CUDA(cudaFuncSetAttribute(conv_out_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    TDX_CHECK_CUDA(cudaFuncSetAttribute(conv_out_kernel<8, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    TDX_CHECK_CUDA(cudaFuncSetAttribute(conv_out_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    TDX_CHECK_CUDA(cudaFuncSetAttribute(conv_out_kernel<8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   }
   return TDX_OK;
 }
@@ -464,7 +478,16 @@ int conv_out_validate(const TdxConvOutDesc& d) {
   return TDX_OK;
 }
 
-int conv_out_launch(const TdxConvOutDesc& d, cudaStream_t stream) {
+int conv_out_guided_validate(const TdxConvOutGuidedDesc& d) {
+  int rc = conv_out_validate(d.base);
+  if (rc != TDX_OK) return rc;
+  TDX_REQUIRE(d.guide_out, "conv_out_guided: null guide_out");
+  TDX_REQUIRE(d.base.sched_coef, "conv_out_guided: the guidance scale is read from sched_coef[4]: sched_coef is required");
+  return TDX_OK;
+}
+
+// guide_out == NULL: the plain kernel (bit-identical to a TdxConvOutDesc launch).
+int conv_out_launch_impl(const TdxConvOutDesc& d, const float* guide_out, cudaStream_t stream) {
   ConvOutParams p;
   p.x = reinterpret_cast<const uint4*>(d.x);
   p.C8 = d.c_in / 8;
@@ -476,6 +499,7 @@ int conv_out_launch(const TdxConvOutDesc& d, cudaStream_t stream) {
   p.coef = d.sched_coef;
   p.sample = d.sample;
   p.x0_prev = d.x0_prev;
+  p.guide_out = guide_out;
   const int wout = d.c_out == 1 ? 1 : 8;
   const int smem = 9 * d.c_in * wout * 4;
   int rc_prep = direct_prepare();
@@ -484,9 +508,20 @@ int conv_out_launch(const TdxConvOutDesc& d, cudaStream_t stream) {
   cudaLaunchConfig_t cfg;
   cudaLaunchAttribute attr[1];
   fill_launch_config(&cfg, attr, grid, dim3(128), smem, stream);
-  if (wout == 1) TDX_CHECK_CUDA(cudaLaunchKernelEx(&cfg, conv_out_kernel<1>, p));
-  else TDX_CHECK_CUDA(cudaLaunchKernelEx(&cfg, conv_out_kernel<8>, p));
+  if (guide_out) {
+    if (wout == 1) TDX_CHECK_CUDA(cudaLaunchKernelEx(&cfg, conv_out_kernel<1, true>, p));
+    else TDX_CHECK_CUDA(cudaLaunchKernelEx(&cfg, conv_out_kernel<8, true>, p));
+  } else {
+    if (wout == 1) TDX_CHECK_CUDA(cudaLaunchKernelEx(&cfg, conv_out_kernel<1, false>, p));
+    else TDX_CHECK_CUDA(cudaLaunchKernelEx(&cfg, conv_out_kernel<8, false>, p));
+  }
   return TDX_OK;
+}
+
+int conv_out_launch(const TdxConvOutDesc& d, cudaStream_t stream) { return conv_out_launch_impl(d, nullptr, stream); }
+
+int conv_out_guided_launch(const TdxConvOutGuidedDesc& d, cudaStream_t stream) {
+  return conv_out_launch_impl(d.base, d.guide_out, stream);
 }
 
 // ------------------------------------------------------------------------------------------------ embedding vectors
@@ -763,6 +798,13 @@ extern "C" int tdx_conv_out_run(const TdxConvOutDesc* d, void* stream) {
   int rc = conv_out_validate(*d);
   if (rc != TDX_OK) return rc;
   return conv_out_launch(*d, reinterpret_cast<cudaStream_t>(stream));
+}
+
+extern "C" int tdx_conv_out_guided_run(const TdxConvOutGuidedDesc* d, void* stream) {
+  if (!d) { set_error("conv_out_guided: null descriptor"); return TDX_E_INVALID; }
+  int rc = conv_out_guided_validate(*d);
+  if (rc != TDX_OK) return rc;
+  return conv_out_guided_launch(*d, reinterpret_cast<cudaStream_t>(stream));
 }
 
 extern "C" int tdx_embed_run(const TdxEmbedDesc* d, void* stream) {

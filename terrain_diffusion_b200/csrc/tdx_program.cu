@@ -14,6 +14,8 @@ int im2col_validate(const TdxIm2colDesc& d);
 int im2col_launch(const TdxIm2colDesc& d, cudaStream_t stream);
 int conv_out_validate(const TdxConvOutDesc& d);
 int conv_out_launch(const TdxConvOutDesc& d, cudaStream_t stream);
+int conv_out_guided_validate(const TdxConvOutGuidedDesc& d);
+int conv_out_launch_impl(const TdxConvOutDesc& d, const float* guide_out, cudaStream_t stream);
 int embed_validate(const TdxEmbedDesc& d);
 int direct_prepare();
 int attn_validate(const TdxAttnDesc& d);
@@ -29,6 +31,7 @@ struct Op {
   CUtensorMap tms[3];
   TdxConvInDesc ci;
   TdxConvOutDesc co;
+  const float* guide_out = nullptr;   // OP_CONV_OUT with two-model guidance (tdx_program_add_conv_out_guided)
   TdxEmbedDesc em;
   TdxAttnDesc at;
   TdxIm2colDesc im;
@@ -50,7 +53,7 @@ static int launch_all(TdxProgram* p, cudaStream_t stream) {
     switch (op.type) {
       case OP_CONV_IN: rc = conv_in_launch(op.ci, stream); break;
       case OP_IGEMM: rc = igemm_launch(op.ig, op.tms, stream); break;
-      case OP_CONV_OUT: rc = conv_out_launch(op.co, stream); break;
+      case OP_CONV_OUT: rc = conv_out_launch_impl(op.co, op.guide_out, stream); break;
       case OP_EMBED:
         op.em.blocks = op.blocks.data();
         rc = embed_launch(op.em, stream);
@@ -125,6 +128,20 @@ extern "C" int tdx_program_add_conv_out(TdxProgram* p, const TdxConvOutDesc* d) 
   Op op;
   op.type = OP_CONV_OUT;
   op.co = *d;
+  p->ops.push_back(op);
+  return invalidate_graph(p);
+}
+
+extern "C" int tdx_program_add_conv_out_guided(TdxProgram* p, const TdxConvOutGuidedDesc* d) {
+  TDX_REQUIRE(p && d, "program_add_conv_out_guided: null argument");
+  int rc = conv_out_guided_validate(*d);
+  if (rc != TDX_OK) return rc;
+  rc = direct_prepare();
+  if (rc != TDX_OK) return rc;
+  Op op;
+  op.type = OP_CONV_OUT;
+  op.co = d->base;
+  op.guide_out = d->guide_out;
   p->ops.push_back(op);
   return invalidate_graph(p);
 }
@@ -218,7 +235,7 @@ extern "C" int tdx_program_profile(TdxProgram* p, float* ms_per_launch, int32_t*
     switch (op.type) {
       case OP_CONV_IN: rc = conv_in_launch(op.ci, stream); break;
       case OP_IGEMM: rc = igemm_launch(op.ig, op.tms, stream); break;
-      case OP_CONV_OUT: rc = conv_out_launch(op.co, stream); break;
+      case OP_CONV_OUT: rc = conv_out_launch_impl(op.co, op.guide_out, stream); break;
       case OP_EMBED:
         op.em.blocks = op.blocks.data();
         rc = embed_launch(op.em, stream);

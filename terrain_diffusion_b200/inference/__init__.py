@@ -1,6 +1,7 @@
 """Mirror of the sampling part of terrain_diffusion.inference / terrain_diffusion.training.evaluation."""
 from .canvas import BlendCanvas  # noqa: F401
-from .samplers import (sample_decoder_consistency_tiled, sample_decoder_diffusion_sharded,  # noqa: F401
+from .samplers import (process_base_cond_img, sample_base_diffusion,  # noqa: F401
+                       sample_decoder_consistency_tiled, sample_decoder_diffusion_sharded,
                        sample_decoder_diffusion_tiled)
 from .sharded import ShardedCanvas  # noqa: F401
 from .solve import DiffusionSolve  # noqa: F401

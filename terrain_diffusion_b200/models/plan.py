@@ -300,6 +300,7 @@ class UNetEmitter:
         self.conv_in_direct = os.environ.get("TDX_CONV_IN_DIRECT") == "1"
         self.arena: dict = {}
         self.cvecs: dict = {}
+        self.igemm_flops = 0          # sum of 2*M*N*K over the igemm launches this emitter has appended
 
     def act(self, key, c, h, w):
         if key not in self.arena:
@@ -417,6 +418,8 @@ class UNetEmitter:
     def _add_igemm(self, prog, d):
         self._apply_tuned_shape(d)
         L.check(L.lib().tdx_program_add_igemm(prog.handle, C.byref(d)))
+        k = sum(d.a_channels[i] * d.a_taps[i] for i in range(d.n_seg))
+        self.igemm_flops += 2 * d.n_img * d.height * d.width * d.c_out * k
         prog.n_igemm += 1
         prog.n_launch += 1
 
@@ -556,7 +559,8 @@ class UNetEmitter:
 
     def _emit(self, prog: UNetProgram, srcs, model_out=None, sched=None, cvec_set: int = 0):
         """srcs: [(tensor NCHW fp32/bf16, channels, scale_ptr_tensor or None)] (1 or 2 sources);
-        model_out: fp32 [n, Cout, h, w] or None; sched: None or dict(coef=tensor[4], sample=tensor, x0_prev=tensor);
+        model_out: fp32 [n, Cout, h, w] or None; sched: None or dict(coef=tensor[4], sample=tensor, x0_prev=tensor)
+        or, for two-model guidance, dict(coef=tensor[5] {.., s}, sample=, x0_prev=, guide_out=fp32 [n, Cout, h, w]);
         cvec_set: which label set's modulation vectors (see emit_embed) this evaluation uses."""
         fw = self.fw
         g = fw.g
@@ -682,7 +686,13 @@ class UNetEmitter:
             od.sched_coef = sched["coef"].data_ptr()
             od.sample = sched["sample"].data_ptr()
             od.x0_prev = sched["x0_prev"].data_ptr()
-        L.check(L.lib().tdx_program_add_conv_out(prog.handle, C.byref(od)))
+        if sched is not None and sched.get("guide_out") is not None:
+            gd = L.TdxConvOutGuidedDesc()
+            gd.base = od
+            gd.guide_out = sched["guide_out"].data_ptr()
+            L.check(L.lib().tdx_program_add_conv_out_guided(prog.handle, C.byref(gd)))
+        else:
+            L.check(L.lib().tdx_program_add_conv_out(prog.handle, C.byref(od)))
         prog.n_launch += 1
         prog.keep.append((self.arena, self.cvecs, fw, srcs, model_out, sched))
         prog.arena = self.arena
